@@ -18,6 +18,9 @@ ring of input frames larger than L2, so no launch finds its source in cache.
 `--impl reference` times the reference CPU path instead (oracle port; the Rust original cannot be built: no rustc).
 Side measurements (not the headline): --config 1/3/31/4 (the other BASELINE configurations), --interp (other resamplers),
 --lens (other lens models), --planes N (multi-plane frames through gf_cuda_undistort_planes_dev).
+
+`--dump-outputs DIR` writes what the timed path rendered in its last timed step to DIR (see OutputSample), so that two builds
+run with the same arguments (hence the same seeded inputs) can be compared output for output.
 """
 import argparse
 import ctypes as C
@@ -166,6 +169,49 @@ def make_mesh():
     return synth.synthetic_mesh(W, H) if CFG.get("mesh") else None
 
 
+DUMP_MAX_VALUES = 12 << 20      # float32 values in frames.npy (48 MB) plus at most 1 Mi float64 sample indices (8 MB): under 64 MB
+DUMP_SEED = 20240917
+
+
+class OutputSample:
+    """--dump-outputs: the output buffers the last timed step left behind, as pixel elements (uint8 / uint16 / f16 / f32, all
+    exact in float32).  A buffer's image area (rows x row_bytes, stride padding excluded) is kept whole when it fits, otherwise
+    at one fixed, seeded set of element positions, the same for every run and build with the same arguments.
+      frames.npy        float32 [buffers, n]: the sampled elements of each buffer, oldest frame first
+      sample_index.npy  float64 [n]: their row-major element indices inside the image area"""
+
+    def __init__(self, rows, row_bytes, pix, n_bufs):
+        from gyroflow_b200 import abi
+        self.rows, self.row_bytes, self.dtype = rows, row_bytes, np.dtype(abi.PIXEL_TYPES[pix][2])
+        total = rows * row_bytes // self.dtype.itemsize
+        n = min(total, DUMP_MAX_VALUES // n_bufs, 1 << 20)
+        self.index = np.arange(total) if n == total else np.sort(np.random.default_rng(DUMP_SEED).choice(total, n, replace=False))
+        self.byte_index = (self.index[:, None] * self.dtype.itemsize + np.arange(self.dtype.itemsize)).reshape(-1)
+        self.samples = []
+
+    def take(self, bufs):
+        """bufs: rows x stride uint8 buffers, numpy arrays or torch tensors (gathered on their device: no full-frame copy)."""
+        for b in bufs:
+            idx = self.byte_index
+            if not isinstance(b, np.ndarray):
+                import torch
+                idx = torch.from_numpy(idx).to(b.device)
+            self.samples.append(b[:self.rows, :self.row_bytes].reshape(-1)[idx])
+
+    def write(self, out_dir):
+        os.makedirs(out_dir, exist_ok=True)
+        host = [s if isinstance(s, np.ndarray) else s.cpu().numpy() for s in self.samples]
+        np.save(os.path.join(out_dir, "frames.npy"), np.stack([np.ascontiguousarray(h).view(self.dtype) for h in host]).astype(np.float32))
+        np.save(os.path.join(out_dir, "sample_index.npy"), self.index.astype(np.float64))
+
+
+def last_step_slots(step, planes=1):
+    """Ring slots holding the frames of `step` that are still resident after it (frame i of the run lives in slot i % RING, its
+    planes in slots (i % RING) * planes + k), oldest first."""
+    last = range((step + 1) * FRAMES_PER_STEP - min(RING, FRAMES_PER_STEP), (step + 1) * FRAMES_PER_STEP)
+    return [(i % RING) * planes + k for i in last for k in range(planes)]
+
+
 def cpu_reference_fps(p, mats, frames, threads):
     """The reference's CPU path (oracle port) on `frames` full 4K frames, all host threads."""
     from gyroflow_b200 import synth
@@ -199,6 +245,10 @@ def run_reference(args):
     for i in range(args.steps): assert step(i) == 0
     dt = time.perf_counter() - t0
     fps = args.steps / dt
+    if args.dump_outputs:
+        sample = OutputSample(H, W * p.bytes_per_pixel, PIX, 1)
+        sample.take([dst])
+        sample.write(args.dump_outputs)
     print(json.dumps({
         "impl": "reference", "metric": METRIC, "value": fps, "unit": "frames/s", "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
         "ms_per_step": dt / args.steps * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
@@ -285,6 +335,10 @@ def run_pipeline(args, torch, dist, g, rank, world, local, dev):
     e1.record(tstream)
     torch.cuda.synchronize()
     clocks.mark_end()
+    sample = None
+    if args.dump_outputs and rank == 0:                   # before any further step overwrites the ring
+        sample = OutputSample(H, W * p.bytes_per_pixel, PIX, min(RING, FRAMES_PER_STEP))
+        sample.take([frames_out[k] for k in last_step_slots(W_STEPS + args.steps - 1)])
     if world > 1: dist.barrier()
     total_ms = e0.elapsed_time(e1)
     launches = q.launch_count - l0
@@ -469,6 +523,7 @@ def run_pipeline(args, torch, dist, g, rank, world, local, dev):
                          "note": "kernel is FP32-issue bound in bit-exact (-fmad=false) mode, not HBM bound; traffic is the DRAM bytes of ONE cold launch under ncu (output stays in L2), not a steady-state figure; see DESIGN.md"},
             "cpu_baseline": cpu,
         }
+        if sample: sample.write(args.dump_outputs)
         print(json.dumps(out))
     ctx.close(); dg.close(); q.close()
     if world > 1:
@@ -491,6 +546,8 @@ def main():
     ap.add_argument("--digital", default=None, help="override the config's digital lens (side measurement), e.g. gopro_superview, digital_stretch, gopro_warp")
     ap.add_argument("--planes", type=int, default=1, help="planes of this geometry per frame, rendered by one gf_cuda_undistort_planes_dev call (side measurement)")
     ap.add_argument("--interp", default="Bilinear", help="Bilinear (BASELINE), Bicubic, Lanczos4, 'EWA: Robidoux', ... (side measurement)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the frames the last timed step rendered (rank 0's; a fixed seeded sample) to DIR/frames.npy + DIR/sample_index.npy")
     args = ap.parse_args()
     select_config(args.config)
     global INTERP, LENS, WORKLOAD
@@ -592,6 +649,11 @@ def main():
         ev[s][1].record(tstream)
     torch.cuda.synchronize()
     clocks.mark_end()
+    sample = None
+    if args.dump_outputs and rank == 0:                   # before any further step overwrites the ring
+        slots = last_step_slots(args.steps - 1, NPL)
+        sample = OutputSample(BH, BW * p.bytes_per_pixel, PIX, len(slots))
+        sample.take([frames_out[k] for k in slots])
     if world > 1: dist.barrier()
     total_ms = sum(a.elapsed_time(b) for a, b in ev)
     launches = ctx.launch_count - l0
@@ -679,6 +741,7 @@ def main():
                          "note": "kernel is FP32-issue bound in bit-exact (-fmad=false) mode; see DESIGN.md"},
             "cpu_baseline": cpu,
         }
+        if sample: sample.write(args.dump_outputs)
         print(json.dumps(out))
     for c in hctx: c.close()
     ctx.close()
