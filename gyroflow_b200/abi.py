@@ -198,6 +198,7 @@ EXPORTS = [
     ("gf_cuda_last_error", C.c_char_p, [C.c_void_p]),
     ("gf_cuda_backend_name", C.c_char_p, []),
     ("gf_cuda_launch_count", C.c_uint64, [C.c_void_p]),
+    ("gf_cuda_filter_counts", C.c_int, [C.c_void_p, C.POINTER(C.c_uint32)]),
     ("gf_cuda_selftest", C.c_int, [C.c_int, C.c_ulonglong, C.c_ulonglong, _P(C.c_ulonglong)]),
     ("gf_frame_transform_at_timestamp", C.c_int, [_P(ComputeParams), C.c_double, C.c_size_t, _P(KernelParams), C.c_void_p, C.c_size_t,
                                                   _P(C.c_size_t), _P(C.c_double), _P(C.c_double)]),

@@ -207,6 +207,15 @@ class CudaWrapper:
     def launch_count(self):
         return int(self._lib.gf_cuda_launch_count(self._h))
 
+    def filter_counts(self):
+        """Counters of the latest frame on the filtered rolling-shutter pre-pass (waits for the work queued so far): pairs and pixels
+        sent to the tail launch, whether a queue was full, and how many of the pairs the final pass deferred (gf_cuda_filter_counts)."""
+        out = (C.c_uint32 * 4)()
+        rc = self._lib.gf_cuda_filter_counts(self._h, out)
+        if rc != 0:
+            raise self._err(rc)
+        return dict(pairs=int(out[0]), pixels=int(out[1]), overflow=bool(out[2]), bad_pairs=int(out[3]))
+
     def close(self):
         if self._h:
             self._lib.gf_cuda_destroy(self._h)

@@ -47,11 +47,14 @@ struct gf_cuda_ctx {
     KernelFn fn_lean = nullptr;   // rare features compiled out
     KernelFn fn_x2 = nullptr;     // lean + two pixels per thread on the packed f32x2 pipe; trusted / guarded path picked from a device word
     KernelFn fn_x2c = nullptr;    // the packed kernel writing a coordinate map (pass 1 of the two-pass path)
+    KernelFn fn_x2f = nullptr;    // the packed kernel's main launch for filtered frames (fn_x2 renders their tail)
     uint32_t* d_const_flags = nullptr;   // two device words {0, 1}: the verdict of the host scan of host tables, as the kernel wants it
     uint32_t* d_vflags = nullptr;        // scratch verdict word of gf_cuda_validate_tables_dev
     cudaStream_t last_stream = nullptr;  // the stream of the most recent call (gf_cuda_synchronize waits for it too)
-    // filtered rolling-shutter pre-pass (packed fisheye kernel): queue of deferred pixel pairs + two ping-pong counters
-    uint32_t* d_defer_q = nullptr; unsigned* d_defer_count = nullptr; uint32_t defer_cap = 0; unsigned long long filter_frames = 0;
+    // filtered rolling-shutter pre-pass (packed fisheye kernel): queues of deferred pixel pairs and pixels + two ping-pong sets of
+    // GF_FLT_WORDS counters; defer_cap / defer_cap_px: queue capacities, GF_X2_DEFER_CAP overrides both (tests of the full-queue path)
+    uint32_t* d_defer_q = nullptr; uint4* d_defer_px = nullptr; unsigned* d_defer_count = nullptr;
+    uint32_t defer_cap = 1u << 20, defer_cap_px = 1u << 20; unsigned long long filter_frames = 0;
     bool no_filter = false;
     int block_y = GF_BLOCK_Y, x2_block_y = 4;   // tuning knobs GF_BLOCK_Y / GF_X2_BLOCK_Y, read once per context at creation
     // preview overlays (overlay.cu), off unless gf_cuda_set_overlays: device copy of the drawing buffer, private copy of a DEVICE input
@@ -405,10 +408,12 @@ GF_API int gf_cuda_create(gf_cuda_ctx** out_ctx, int device, const gf_kernel_par
     ctx->device = device; ctx->pixel_type = pixel_type; ctx->distortion_model = distortion_model; ctx->digital_lens = digital_lens;
     ctx->interpolation = params->interpolation; ctx->layout = layout; ctx->bpp = bpp; ctx->fn = fn; ctx->fn_lean = fn_lean; ctx->fn_x2 = fn_x2; ctx->fn_shade = gf_shade_kernel(layout);
     if (!no_x2) ctx->fn_x2c = find_kernel(distortion_model, digital_lens, layout, GF_INTERP_BILINEAR, 4);
+    if (!no_x2) ctx->fn_x2f = find_kernel(distortion_model, digital_lens, layout, params->interpolation, 5);
     ctx->width = params->width; ctx->height = params->height; ctx->output_width = params->output_width; ctx->output_height = params->output_height;
     ctx->drawing_len = drawing_len; ctx->no_filter = no_filter;
     { const char* e = getenv("GF_BLOCK_Y"); const int v = e ? atoi(e) : GF_BLOCK_Y; ctx->block_y = (v == 1 || v == 2 || v == 4 || v == 8) ? v : GF_BLOCK_Y; }
     { const char* e = getenv("GF_X2_BLOCK_Y"); const int v = e ? atoi(e) : 4; ctx->x2_block_y = (v == 1 || v == 2 || v == 4 || v == 8) ? v : 4; }
+    { const char* e = getenv("GF_X2_DEFER_CAP"); const long v = e ? atol(e) : 0; if (v > 0 && v < (1l << 20)) ctx->defer_cap = ctx->defer_cap_px = (uint32_t)v; }
     auto bail = [&](int rc) { std::string m = ctx->last_error; gf_cuda_destroy(ctx); g_last_error = m; return rc; };
 
     cudaError_t e = cudaSetDevice(device);
@@ -465,6 +470,7 @@ GF_API void gf_cuda_destroy(gf_cuda_ctx* ctx) {
     if (ctx->d_drawing) cudaFree(ctx->d_drawing);
     if (ctx->d_src_ovl) cudaFree(ctx->d_src_ovl);
     if (ctx->d_defer_q) cudaFree(ctx->d_defer_q);
+    if (ctx->d_defer_px) cudaFree(ctx->d_defer_px);
     if (ctx->d_defer_count) cudaFree(ctx->d_defer_count);
     if (ctx->d_coords) cudaFree(ctx->d_coords);
     if (ctx->stream) cudaStreamDestroy(ctx->stream);
@@ -673,24 +679,27 @@ static int run_warp(gf_cuda_ctx* ctx, const gf_buffer_desc* in, const gf_buffer_
         const dim3 block2(GF_BLOCK_X, by), grid2(grid.x, (A.out_rows + 2 * by - 1) / (2 * by));
         // filtered pre-pass: fisheye without a digital lens, rolling shutter on, geometry that fits the queue's 16 + 16 bit entries
         const float a_cap = (ctx->distortion_model == GF_LENS_OPENCV_FISHEYE && ctx->digital_lens == GF_LENS_NONE && (A.feat & F_RS) && !ctx->no_filter &&
-                             A.out_cols <= 65536 && A.out_rows <= 131072 &&
+                             A.out_cols <= 65536 && A.out_rows <= 131072 && (two_pass || ctx->fn_x2f) &&
                              (tables_on_device || table_flags == 0)) ? filter_a_cap(p->k) : 0.0f;      // host tables known to be wild / IBIS: guarded path, no tail launch
         if (a_cap > 0.0f) {
             if (!ctx->d_defer_q) {
-                ctx->defer_cap = 1u << 20;                             // 4 MB: 1 M pairs = a quarter of a 4K frame's pairs; a full queue falls back inline
+                // 1 M pairs (4 MB, a quarter of a 4K frame's pairs) and 1 M pixels (16 MB, an eighth of a 4K frame); a full queue costs
+                // the frame a second, exact rendering in the tail launch (COORD frames: the pairs past the end take the exact pre-pass inline)
                 CK(cudaMalloc(&ctx->d_defer_q, (size_t)ctx->defer_cap * sizeof(uint32_t)));
-                CK(cudaMalloc(&ctx->d_defer_count, 2 * sizeof(unsigned)));
-                CK(cudaMemsetAsync(ctx->d_defer_count, 0, 2 * sizeof(unsigned), st));
+                CK(cudaMalloc(&ctx->d_defer_px, (size_t)ctx->defer_cap_px * sizeof(uint4)));
+                CK(cudaMalloc(&ctx->d_defer_count, 2 * GF_FLT_WORDS * sizeof(unsigned)));
+                CK(cudaMemsetAsync(ctx->d_defer_count, 0, 2 * GF_FLT_WORDS * sizeof(unsigned), st));
             }
             const unsigned cur = (unsigned)(ctx->filter_frames & 1ull);
             ctx->filter_frames++;
             A.feat |= F_FILTER;
             A.flt.q = ctx->d_defer_q; A.flt.cap = ctx->defer_cap;
-            A.flt.count = ctx->d_defer_count + cur; A.flt.count_next = ctx->d_defer_count + (cur ^ 1u);
+            A.flt.qpx = ctx->d_defer_px; A.flt.cap_px = ctx->defer_cap_px;
+            A.flt.count = ctx->d_defer_count + cur * GF_FLT_WORDS; A.flt.count_next = ctx->d_defer_count + (cur ^ 1u) * GF_FLT_WORDS;
             A.flt.rho = 0x1p-17f; A.flt.a_cap = a_cap; A.flt.tail = 0;
-            CK(launch_pdl(x2, grid2, block2, A)); ctx->x2_launches++;
-            A.flt.tail = 1;                                            // the deferred pairs, exact pre-pass; also re-arms the other counter
-            // one thread per deferred pair for up to 2 % of a 4K frame's pairs in a single wave of tiny blocks (idle blocks exit at once);
+            CK(launch_pdl(two_pass ? x2 : ctx->fn_x2f, grid2, block2, A)); ctx->x2_launches++;
+            A.flt.tail = 1;                                            // the deferred pairs and pixels; also re-arms the other counters
+            // one thread per deferred entry for up to 2 % of a 4K frame's pairs in a single wave of tiny blocks (idle blocks exit at once);
             // more entries than threads are covered by the grid-stride loop
             CK(launch_pdl(x2, dim3(148 * 16, 1), block2, A));
             ctx->launches++;
@@ -1033,5 +1042,14 @@ GF_API int gf_cuda_set_overlays(gf_cuda_ctx* ctx, int enabled) {
 
 GF_API const char* gf_cuda_last_error(gf_cuda_ctx* ctx) { return ctx ? ctx->last_error.c_str() : g_last_error.c_str(); }
 GF_API uint64_t gf_cuda_launch_count(gf_cuda_ctx* ctx) { return ctx ? ctx->launches : 0; }
+GF_API int gf_cuda_filter_counts(gf_cuda_ctx* ctx, uint32_t* out) {
+    if (!ctx || !out) return fail(ctx, GF_ERR_BAD_PARAMS, "null argument");
+    memset(out, 0, GF_FLT_WORDS * sizeof(uint32_t));
+    if (ctx->filter_frames == 0) return GF_OK;
+    { const int rc = gf_cuda_synchronize(ctx); if (rc != GF_OK) return rc; }
+    const unsigned cur = (unsigned)((ctx->filter_frames - 1) & 1ull);     // the latest frame's set: the next one zeroes the other
+    CK(cudaMemcpy(out, ctx->d_defer_count + cur * GF_FLT_WORDS, GF_FLT_WORDS * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+    return GF_OK;
+}
 
 } // extern "C"

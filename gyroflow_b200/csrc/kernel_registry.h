@@ -37,6 +37,7 @@ KernelFn gf_kernel_generic_polynomial(int digital, int layout, int interp, int l
 KernelFn gf_kernel_gopro(int digital, int layout, int interp, int lean);
 KernelFn gf_shade_kernel(int layout);      // pass 2 of the multi-plane mode (shade_kernel.cu)
 
+// lean == 5: the packed kernel's filtered instantiation (FILTERED in warp_kernel_x2.cuh), where the lens model has an approximate form
 // lean == 4: the packed kernel in coordinate-output mode (pass 1 of the two-pass path); one instantiation per lens model serves
 // every pixel layout
 // lean == 2: the two-pixels-per-thread packed-f32x2 kernel (warp_kernel_x2.cuh), where the lens model has a packed form; it carries
@@ -45,13 +46,19 @@ template <int LENS, int DIGITAL, class PIX>
 static KernelFn pick_x2(int interp) {
     // packed digital lenses: superview, superview6, hyperview (fisheye pairs) and digital_stretch (every packed lens model)
     if constexpr (Lens2<LENS>::kHas && Digital2<DIGITAL>::kHas) {
-        // 6 resident blocks per SM (40 registers): 5 (48 registers, no spills) measured the same, 4 slower, 7 / 8 compile to the 6 code
+        // 6 resident blocks per SM (40 registers): 5 (48 registers) measured 2 % slower on the filtered headline frames, 4 slower still,
+        // 7 / 8 compile to the 6 code
         if (interp == GF_INTERP_BILINEAR) return warp_kernel_x2<LENS, DIGITAL, PIX, GF_X2_MINB>;
     }
     return nullptr;
 }
 template <int LENS, int DIGITAL, class PIX>
 static KernelFn pick_interp(int interp, int lean) {
+    if (lean == 5) {        // the packed kernel's main launch for filtered frames (fused bilinear sampling)
+        if constexpr (LensApprox<LENS>::value && DIGITAL == GF_LENS_NONE)
+            if (interp == GF_INTERP_BILINEAR) return warp_kernel_x2<LENS, DIGITAL, PIX, GF_X2_MINB, false, true>;
+        return nullptr;
+    }
     if (lean == 4) {
         if constexpr (Lens2<LENS>::kHas && Digital2<DIGITAL>::kHas)
             return warp_kernel_x2<LENS, DIGITAL, Pix<1, SC_U8>, GF_X2_MINB, true>;

@@ -70,6 +70,15 @@ template <bool GEN> __device__ __forceinline__ bool has(uint32_t feat, uint32_t 
     return (feat & bit) != 0;        // F_RS, F_IS_Y stay dynamic
 }
 
+// per-frame counters of the filtered pre-pass (WarpArgs::X2Filter::count); appends are counted even when the queue is full
+enum {
+    GF_FLT_PAIRS    = 0,      // pairs appended to the deferred-pair queue (uncertified row or `bad`)
+    GF_FLT_PIXELS   = 1,      // pixels appended to the deferred-pixel queue
+    GF_FLT_OVERFLOW = 2,      // non-zero: a queue was full, the tail launch re-renders the whole frame
+    GF_FLT_BAD      = 3,      // of GF_FLT_PAIRS, the pairs deferred because the final pass set `bad`
+    GF_FLT_WORDS    = 4
+};
+
 struct WarpArgs {
     gf_kernel_params p;             // verbatim KernelParams
     const uint8_t* src;
@@ -81,14 +90,16 @@ struct WarpArgs {
     uint2*         coord_out;       // multi-plane mode, pass 1: write the source coordinates of every output pixel here instead of sampling
     const uint2*   coord_in;        // pass 2 (shade_from_coords_kernel): read them back
     const uint32_t* table_flags;    // device word: 0 = the matrix table is tame and IBIS-free (packed kernel: trusted path), see warp_kernel_x2
-    // filtered rolling-shutter pre-pass of the packed kernel (F_FILTER): pairs whose row choice the approximate evaluation cannot
-    // certify are appended to `q` and rendered by a second launch of the same kernel in tail mode
+    // filtered rolling-shutter pre-pass of the packed kernel (F_FILTER): the main launch appends what it does not finish to two queues
+    // (pairs whose row choice the approximate evaluation cannot certify or whose fast sequences left their window; pixels whose 8-bit
+    // footprint is not interior) and a second launch of the kernel in tail mode renders them
     struct X2Filter {
         uint32_t* q;                // deferred pairs: x | (y0 / 2) << 16
-        unsigned* count;            // number of entries appended by this frame's main launch
-        unsigned* count_next;       // the next frame's counter, zeroed by this frame's tail launch
-        uint32_t  cap;              // capacity of q (a full queue makes the thread take the exact pre-pass inline)
-        int       tail;             // 1 = this launch renders the queue
+        uint4*    qpx;              // deferred pixels: {x, y, bits(u), bits(v)}, u and v exact
+        unsigned* count;            // this frame's GF_FLT_WORDS counters (GF_FLT_* above)
+        unsigned* count_next;       // the next frame's counters, zeroed by this frame's tail launch
+        uint32_t  cap, cap_px;      // capacities of q and qpx (COORD frames: a full q makes the thread take the exact pre-pass inline)
+        int       tail;             // 1 = this launch renders the queues
         float     rho;              // relative tolerance of the certificate
         float     a_cap;            // r^2 below which the tolerance holds for this lens (polynomial conditioning), <= 2^14
     } flt;

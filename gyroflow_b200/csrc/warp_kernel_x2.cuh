@@ -550,10 +550,36 @@ static __device__ __noinline__ void shade_cold(bool ok, float u, float v, const 
     PIX::store(out, true, pixel);
 }
 
-// sampling + conversion + store of one pixel, lean feature set (no fix_range, background mode 0, pixel_value_limit >= max).
-// wu, wv: round_half_away_w of 64 * u, 64 * v (8-bit formats only).
-template <class PIX>
-GF_DEV void shade_lean(bool ok, bool far, float u, float v, int wu, int wv, const WarpArgs& A, uint8_t* __restrict__ out) {
+// warp-aggregated atomicAdd(counter, 1) over the active lanes (one atomic per warp); returns this lane's slot.  blockDim.x == 32.
+GF_DEV unsigned warp_append(unsigned* counter) {
+    const unsigned m = __activemask();
+    const unsigned lane = threadIdx.x & 31u;
+    const int leader = __ffs((int)m) - 1;
+    unsigned base = 0;
+    if ((int)lane == leader) base = atomicAdd(counter, (unsigned)__popc(m));
+    base = __shfl_sync(m, base, leader);
+    return base + (unsigned)__popc(m & ((1u << lane) - 1u));
+}
+// append the pair (x, y0), y0 even, to the frame's deferred-pair queue; false when the queue is full
+GF_DEV bool defer_pair(const WarpArgs& A, int x, int y0) {
+    const unsigned slot = warp_append(A.flt.count + GF_FLT_PAIRS);
+    if (slot >= A.flt.cap) return false;
+    A.flt.q[slot] = (uint32_t)x | ((uint32_t)(y0 >> 1) << 16);
+    return true;
+}
+// append pixel (x, y) with its exact source coordinates to the frame's deferred-pixel queue; a full queue marks the frame for the
+// tail launch's whole-frame re-render
+GF_DEV void defer_pixel(const WarpArgs& A, int x, int y, float u, float v) {
+    const unsigned slot = warp_append(A.flt.count + GF_FLT_PIXELS);
+    if (slot < A.flt.cap_px) A.flt.qpx[slot] = make_uint4((uint32_t)x, (uint32_t)y, __float_as_uint(u), __float_as_uint(v));
+    else A.flt.count[GF_FLT_OVERFLOW] = 1u;
+}
+
+// sampling + conversion + store of one pixel (x, y), lean feature set (no fix_range, background mode 0, pixel_value_limit >= max).
+// wu, wv: round_half_away_w of 64 * u, 64 * v (8-bit formats only).  DEFER (filtered body): a pixel without an interior 8-bit
+// footprint goes to the deferred-pixel queue, which the tail launch finishes with shade_cold from the same u, v.
+template <class PIX, bool DEFER = false>
+GF_DEV void shade_lean(bool ok, bool far, float u, float v, int wu, int wv, const WarpArgs& A, uint8_t* __restrict__ out, int x, int y) {
     constexpr int C = PIX::COUNT;
     if (PIX::SCALAR == SC_U8) {
         const int sx0 = wu >> 1, sy0 = wv >> 1;
@@ -566,6 +592,8 @@ GF_DEV void shade_lean(bool ok, bool far, float u, float v, int wu, int wv, cons
             #pragma unroll
             for (int ch = 0; ch < C; ++ch) s[ch] = N[ch] >> 10;      // trunc(N / 1024); N / 1024 <= 255 <= pixel_value_limit
             PIX::store_scalars(out, true, s);
+        } else if (DEFER) {
+            defer_pixel(A, x, y, u, v);
         } else {
             shade_cold<PIX>(ok, u, v, A, out);
         }
@@ -587,9 +615,13 @@ GF_DEV void shade_lean(bool ok, bool far, float u, float v, int wu, int wv, cons
 // pixel size then comes from KernelParams, PIX is a placeholder).
 // exact_prepass: evaluate the mid-row transform with the reference's own arithmetic (always true unless the frame runs the filtered
 // pre-pass; true as well for the pairs the tail launch re-renders)
-template <int LENS, int DIGITAL, class PIX, bool TRUSTED, bool COORD>
+// FILTERED: the main launch of a filtered frame (trusted tables, fused sampling).  Everything rare leaves the launch instead of running
+// inline, so the body holds no call: an uncertified row or a `bad` pair goes to the deferred-pair queue (neither pixel written), a
+// pixel without an interior 8-bit footprint to the deferred-pixel queue, and a full queue to the tail's whole-frame re-render.
+template <int LENS, int DIGITAL, class PIX, bool TRUSTED, bool COORD, bool FILTERED = false>
 GF_DEV void warp_x2_body(const WarpArgs& A, const int x, const int y0, const bool exact_prepass) {
     using namespace p2;
+    static_assert(!FILTERED || (TRUSTED && !COORD && LensApprox<LENS>::value && DIGITAL == GF_LENS_NONE), "filtered body: trusted fused fisheye only");
     const gf_kernel_params& P = A.p;
     if (x >= A.out_cols || y0 >= A.out_rows) return;
     const unsigned long long BYTES = COORD ? (unsigned long long)P.bytes_per_pixel : (unsigned long long)PIX::BYTES;
@@ -628,7 +660,7 @@ GF_DEV void warp_x2_body(const WarpArgs& A, const int x, const int y0, const boo
     int sy_a, sy_b;
     round_away_clamped_x2(py, lim, sy_a, sy_b);                                                         // :465-469
     bool have_row = false;
-    if constexpr (TRUSTED && LensApprox<LENS>::value && DIGITAL == GF_LENS_NONE) if (!exact_prepass) {  // F_FILTER & F_RS (host)
+    if constexpr (TRUSTED && LensApprox<LENS>::value && DIGITAL == GF_LENS_NONE) if (FILTERED || !exact_prepass) {  // F_FILTER & F_RS (host)
         // :470-479, filtered: certify round(v_mid) from the approximate evaluation, defer the pair when it cannot be
         const MatRow9 rm = load_row9(A.matrices, (uint32_t)P.matrix_count / 2u);
         const float bx = pxs * rm.m01.x, by = pxs * rm.m23.y, bw = pxs * rm.m67.x;                      // the reference's products and sums, unfused
@@ -647,19 +679,13 @@ GF_DEV void warp_x2_body(const WarpArgs& A, const int x, const int y0, const boo
         if (sure) {
             round_away_clamped_x2(mk(ta, tb), lim, sy_a, sy_b);
             have_row = true;
-        } else {                                         // append the pair to the frame's queue (warp-aggregated), rendered by the tail launch
-            const unsigned m = __activemask();
-            const unsigned lane = threadIdx.x & 31u;
-            const int leader = __ffs((int)m) - 1;
-            unsigned base = 0;
-            if ((int)lane == leader) base = atomicAdd(A.flt.count, (unsigned)__popc(m));
-            base = __shfl_sync(m, base, leader);
-            const unsigned slot = base + (unsigned)__popc(m & ((1u << lane) - 1u));
-            if (slot < A.flt.cap) { A.flt.q[slot] = (uint32_t)x | ((uint32_t)(y0 >> 1) << 16); return; }
+        } else {                                         // append the pair to the frame's queue, rendered by the tail launch
+            if (defer_pair(A, x, y0)) return;
+            if (FILTERED) { A.flt.count[GF_FLT_OVERFLOW] = 1u; return; }
             // queue full: this thread evaluates the exact pre-pass itself
         }
     }
-    if ((A.feat & F_RS) && !have_row) {                                                                 // :470-479
+    if (!FILTERED && (A.feat & F_RS) && !have_row) {                                                    // :470-479
         const uint32_t mid = (uint32_t)P.matrix_count / 2u;
         f2 tu, tv; bool oa = true, ob = true, bad = false;
         rotate_and_distort_x2<LENS, DIGITAL, TRUSTED>(px, py, mid, mid, A, tu, tv, bad);
@@ -677,7 +703,12 @@ GF_DEV void warp_x2_body(const WarpArgs& A, const int x, const int y0, const boo
     rotate_and_distort_x2<LENS, DIGITAL, TRUSTED>(px, py, idx_a, idx_b, A, u, v, bad);                           // :483
     u = map_apply_x2(u, A.smap_x, bad);                                                                 // :510-515
     v = map_apply_x2(v, A.smap_y, bad);
-    if (bad) {
+    if (FILTERED && bad) {                               // the tail renders the pair from scratch
+        warp_append(A.flt.count + GF_FLT_BAD);
+        if (!defer_pair(A, x, y0)) A.flt.count[GF_FLT_OVERFLOW] = 1u;
+        return;
+    }
+    if (!FILTERED && bad) {
         const PairUV c = rotate_and_distort_cold<LENS, DIGITAL>(pxs, py.x, py.y, idx_a, idx_b, A, 1);
         ok_a = (c.ok & 1) != 0; ok_b = (c.ok & 2) != 0; far_a = (c.ok & 4) != 0; far_b = (c.ok & 8) != 0;
         u = mk(c.ua, c.ub); v = mk(c.va, c.vb);
@@ -695,8 +726,18 @@ GF_DEV void warp_x2_body(const WarpArgs& A, const int x, const int y0, const boo
         round_half_away_w<true>(mul(u, bc(64.0f)), wu_a, wu_b);
         round_half_away_w<true>(mul(v, bc(64.0f)), wv_a, wv_b);
     }
-    if (wr_a) shade_lean<PIX>(ok_a, far_a, u.x, v.x, wu_a, wv_a, A, A.dst + off_a);                     // :615-622
-    if (wr_b) shade_lean<PIX>(ok_b, far_b, u.y, v.y, wu_b, wv_b, A, A.dst + off_b);
+    if constexpr (FILTERED) {
+        // the offsets are recomputed here (the empty asm keeps the compiler from reusing the prologue's): kept live from the prologue,
+        // the two 64-bit values were spilled across the whole evaluation under the register cap
+        int xs = x, ys = y0;
+        asm("" : "+r"(xs), "+r"(ys));
+        const unsigned long long o = (unsigned long long)ys * ostride + (unsigned long long)xs * BYTES;
+        if (wr_a) shade_lean<PIX, true>(true, false, u.x, v.x, wu_a, wv_a, A, A.dst + o, xs, ys);       // :615-622
+        if (wr_b) shade_lean<PIX, true>(true, false, u.y, v.y, wu_b, wv_b, A, A.dst + o + ostride, xs, ys + 1);
+    } else {
+        if (wr_a) shade_lean<PIX>(ok_a, far_a, u.x, v.x, wu_a, wv_a, A, A.dst + off_a, x, y0);           // :615-622
+        if (wr_b) shade_lean<PIX>(ok_b, far_b, u.y, v.y, wu_b, wv_b, A, A.dst + off_b, x, y0 + 1);
+    }
 }
 
 // The kernel: both table-trust variants in one launch, selected by a DEVICE word.  `A.table_flags` points to the verdict on the
@@ -705,33 +746,54 @@ GF_DEV void warp_x2_body(const WarpArgs& A, const int x, const int y0, const boo
 // gf_cuda_frame_transform_dev itself): 0 = every entry zero or 2^-40..2^40 and no IBIS rows.  Trust is therefore a property of
 // the bytes the kernel is about to read, ordered by the stream — not of a host-side pointer cache.  The branch is uniform.
 //
-// Filtered frames (F_FILTER, host-selected: trusted-capable lens with an approximate form, rolling shutter on) launch this kernel
-// twice: the main launch certifies each pair's matrix row from the approximate mid-row evaluation and appends the few pairs it
-// cannot certify to a queue; the tail launch (A.flt.tail, a small grid-stride grid) renders exactly those with the exact pre-pass.
-template <int LENS, int DIGITAL, class PIX, int MINB, bool COORD = false>
+// Filtered frames (F_FILTER, host-selected: trusted-capable lens with an approximate form, rolling shutter on) launch two kernels.  The
+// main launch (FILTERED instantiation; COORD: this one) certifies each pair's matrix row from the approximate mid-row evaluation and
+// sends what it cannot finish cheaply to the frame's queues: uncertified and `bad` pairs, and pixels whose 8-bit footprint is not
+// interior.  The tail launch (A.flt.tail, a small grid-stride grid, always this unfiltered instantiation) renders the deferred pairs with
+// the exact pre-pass and finishes the deferred pixels with shade_cold; if a queue overflowed it re-renders the whole frame instead.
+template <int LENS, int DIGITAL, class PIX, int MINB, bool COORD = false, bool FILTERED = false>
 __global__ void __launch_bounds__(GF_BLOCK_X * GF_BLOCK_Y, MINB)
 warp_kernel_x2(const __grid_constant__ WarpArgs A) {
     constexpr bool kFilter = LensApprox<LENS>::value && DIGITAL == GF_LENS_NONE;
     // launched with programmatic stream serialization (c_abi.cu: launch_pdl): nothing of the previous kernel on the stream — the matrix
-    // table and its verdict word, the deferred-pair queue and its counters, the previous frame's output — may be read or written before this
+    // table and its verdict word, the deferred queues and their counters, the previous frame's output — may be read or written before this
     asm volatile("griddepcontrol.wait;" ::: "memory");
     const bool trusted = __ldg(A.table_flags) == 0u;
-    if constexpr (kFilter) if (A.flt.tail) {
+    if constexpr (kFilter && !FILTERED) if (A.flt.tail) {
         const unsigned tid = (blockIdx.y * gridDim.x + blockIdx.x) * (blockDim.x * blockDim.y) + threadIdx.y * blockDim.x + threadIdx.x;
-        if (tid == 0u) *A.flt.count_next = 0u;                       // re-arm the counter the NEXT frame's main launch will use
+        if (tid == 0u) {                                              // re-arm the counters the NEXT frame's main launch will use
+            #pragma unroll
+            for (int i = 0; i < GF_FLT_WORDS; ++i) A.flt.count_next[i] = 0u;
+        }
         if (!trusted) return;                                         // the main launch deferred nothing on the guarded path
-        const unsigned n = min(*A.flt.count, A.flt.cap);
         const unsigned stride = gridDim.x * gridDim.y * blockDim.x * blockDim.y;
-        for (unsigned i = tid; i < n; i += stride) {
-            const uint32_t e = A.flt.q[i];
-            warp_x2_body<LENS, DIGITAL, PIX, true, COORD>(A, (int)(e & 0xffffu), (int)(e >> 16) * 2, true);
+        // a full queue left pixels missing anywhere in the frame: then every pair is rendered, else the deferred pairs, then the pixels
+        const bool all = A.flt.count[GF_FLT_OVERFLOW] != 0u;
+        const unsigned long long cols = (unsigned long long)A.out_cols;
+        const unsigned long long np = all ? cols * (unsigned long long)((A.out_rows + 1) / 2) : min(A.flt.count[GF_FLT_PAIRS], A.flt.cap);
+        const unsigned long long n = np + ((all || COORD) ? 0u : min(A.flt.count[GF_FLT_PIXELS], A.flt.cap_px));
+        for (unsigned long long i = tid; i < n; i += stride) {
+            if (i < np) {
+                int px, py0;
+                if (all) { px = (int)(i % cols); py0 = (int)(i / cols) * 2; }
+                else     { const uint32_t e = A.flt.q[i]; px = (int)(e & 0xffffu); py0 = (int)(e >> 16) * 2; }
+                warp_x2_body<LENS, DIGITAL, PIX, true, COORD>(A, px, py0, true);
+            } else if constexpr (!COORD && PIX::SCALAR == SC_U8) {
+                const uint4 e = A.flt.qpx[i - np];
+                const unsigned long long off = (unsigned long long)e.y * (unsigned long long)A.p.output_stride + (unsigned long long)e.x * PIX::BYTES;
+                shade_cold<PIX>(true, __uint_as_float(e.z), __uint_as_float(e.w), A, A.dst + off);
+            }
         }
         return;
     }
     const int x = blockIdx.x * GF_BLOCK_X + threadIdx.x;
     const int y0 = (blockIdx.y * blockDim.y + threadIdx.y) * 2;          // blockDim.y: the host may launch flatter blocks (GF_X2_BLOCK_Y)
-    if (trusted) warp_x2_body<LENS, DIGITAL, PIX, true, COORD>(A, x, y0, !(kFilter && (A.feat & F_FILTER)));
-    else         warp_x2_body<LENS, DIGITAL, PIX, false, COORD>(A, x, y0, true);
+    if (trusted) {
+        if constexpr (FILTERED) warp_x2_body<LENS, DIGITAL, PIX, true, false, true>(A, x, y0, false);
+        else warp_x2_body<LENS, DIGITAL, PIX, true, COORD>(A, x, y0, !(COORD && kFilter && (A.feat & F_FILTER)));
+    } else {
+        warp_x2_body<LENS, DIGITAL, PIX, false, COORD>(A, x, y0, true);
+    }
 }
 
 } // namespace gf

@@ -315,6 +315,11 @@ GF_API const char* gf_cuda_last_error(gf_cuda_ctx* ctx);     /* ctx may be NULL:
 GF_API const char* gf_cuda_backend_name(void);               /* ProcessedInfo.backend: "CUDA" (mod.rs:195-201) */
 GF_API uint64_t    gf_cuda_launch_count(gf_cuda_ctx* ctx);   /* warp / coordinate / sampling kernels launched by this ctx so far: 1 per bilinear
                                                               * frame, 2 for bicubic / Lanczos4 (coordinate pass + sampling pass), 4 for EWA */
+/* Counters of the most recent frame on the packed fisheye kernel's filtered rolling-shutter pre-pass (waits for the ctx's work first):
+ * out[0] pairs sent to the tail launch (uncertified row choice, or the final pass left the exact fast sequences' window),
+ * out[1] pixels sent to the tail launch (8-bit bilinear footprint not interior), out[2] non-zero if a queue was full (the tail launch
+ * then re-rendered the whole frame), out[3] the part of out[0] deferred by the final pass.  All zero before the first such frame. */
+GF_API int         gf_cuda_filter_counts(gf_cuda_ctx* ctx, uint32_t out[4]);
 
 /* Device self-test of the exact packed-f32x2 primitives (division, square root, atanf, uniform-divisor division)
  * against the scalar IEEE operations they replace: n pseudo-random operand sets, mismatch counts in out4[0..3].
