@@ -7,9 +7,11 @@ from . import abi
 from .abi import KernelParams, BackendMissing, load_library
 from .backend import (BufferDescription, Buffers, FrameTransform, ProcessedInfo, CudaWrapper,
                       GyroflowCoreError, list_devices, ComputeParams, DeviceGyro, zoom_dynamic,
-                      scan_tables_dev, bind_thread_to_device, stab_config, get_frame_transform_at, host_register, host_unregister)
-from .render_queue import RenderQueue
+                      scan_tables_dev, bind_thread_to_device, stab_config, get_frame_transform_at, host_register, host_unregister,
+                      frame_layout, background_for_plane)
+from .render_queue import RenderQueue, FrameRenderQueue
 
 __all__ = ["abi", "KernelParams", "BackendMissing", "load_library", "BufferDescription", "Buffers", "FrameTransform",
            "ProcessedInfo", "CudaWrapper", "GyroflowCoreError", "list_devices", "ComputeParams", "DeviceGyro", "zoom_dynamic",
-           "scan_tables_dev", "bind_thread_to_device", "stab_config", "get_frame_transform_at", "RenderQueue", "host_register", "host_unregister"]
+           "scan_tables_dev", "bind_thread_to_device", "stab_config", "get_frame_transform_at", "RenderQueue", "host_register", "host_unregister",
+           "FrameRenderQueue", "frame_layout", "background_for_plane"]

@@ -131,6 +131,12 @@ class StabConfig(C.Structure):
     ]
 
 
+class PlaneSpec(C.Structure):
+    """gf_plane_spec: one plane of a decoder frame (rendering/mod.rs:563-651): pixel type, size, `yuvi` list, value limit."""
+    _fields_ = [("pixel_type", C.c_int32), ("width", C.c_int32), ("height", C.c_int32), ("n_ind", C.c_int32), ("ind", C.c_int32 * 4),
+                ("max_value", C.c_float)]
+
+
 class QueueConfig(C.Structure):
     _fields_ = [
         ("device", C.c_int32), ("distortion_model", C.c_int32), ("digital_lens", C.c_int32), ("depth", C.c_int32),
@@ -158,6 +164,14 @@ PIXEL_TYPES = {
 }
 
 BUF_NONE, BUF_HOST, BUF_DEVICE = 0, 1, 2
+
+# GF_FRAME_*: the decoder frame formats of rendering/mod.rs:563-651, in the header's order
+FRAME_FORMATS = {name: i for i, name in enumerate([
+    "NV12", "NV21", "P010LE", "P016LE", "P210LE", "P216LE", "P410LE", "P416LE", "YUV420P", "YUVJ420P",
+    "YUV420P10LE", "YUV420P12LE", "YUV420P14LE", "YUV420P16LE", "YUV422P10LE", "YUV422P12LE", "YUV422P14LE", "YUV422P16LE",
+    "YUV444P10LE", "YUV444P12LE", "YUV444P14LE", "YUV444P16LE", "YUVA444P10LE", "YUVA444P12LE", "YUVA444P16LE",
+    "GBRAPF32LE", "GBRPF32LE", "AYUV64LE", "RGB24", "RGBA", "RGB48BE", "RGBA64BE"])}
+FRAME_MAX_PLANES = 4
 
 ERRORS = {0: "Ok", -1: "BadParams", -2: "SizeTooSmall", -3: "SizeMismatch", -4: "InvalidStride",
           -5: "UnsupportedCombo", -6: "CudaError", -7: "BufferTooSmall", -8: "NoStabilizationData"}
@@ -231,6 +245,13 @@ EXPORTS = [
     ("gf_cuda_checksum_dev", C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]),
     ("gf_cuda_host_register", C.c_int, [C.c_void_p, C.c_size_t]),
     ("gf_cuda_host_unregister", C.c_int, [C.c_void_p]),
+    ("gf_frame_layout", C.c_int, [C.c_int, C.c_int32, C.c_int32, _P(PlaneSpec), _P(C.c_size_t)]),
+    ("gf_background_for_plane", C.c_int, [C.c_int, _P(C.c_float), _P(C.c_int32), C.c_size_t, C.c_int, _P(C.c_float)]),
+    ("gf_cuda_queue_create_frame", C.c_int, [_P(C.c_void_p), _P(QueueConfig), _P(ComputeParams), C.c_int, C.c_int, C.c_size_t,
+                                             _P(BufferDesc), _P(BufferDesc)]),
+    ("gf_cuda_queue_submit_frame", C.c_int, [C.c_void_p, C.c_size_t, C.c_double, C.c_size_t, _P(BufferDesc), _P(BufferDesc),
+                                             C.c_void_p, C.c_size_t, C.c_int]),
+    ("gf_cuda_queue_wait_frame", C.c_int, [C.c_void_p, _P(C.c_size_t), _P(C.c_uint64), C.c_size_t]),
 ]
 
 _lib = None

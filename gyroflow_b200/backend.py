@@ -475,3 +475,27 @@ def get_frame_transform_at(stab: abi.StabConfig, cp: ComputeParams, buffers: Buf
     if rc != 0:
         raise GyroflowCoreError(rc, "gf_get_frame_transform_at")
     return kernel_params
+
+
+PIXEL_TYPE_NAMES = {v[0]: k for k, v in abi.PIXEL_TYPES.items()}
+
+
+def frame_layout(format: str, width: int, height: int):
+    """The planes of a width x height decoder frame (gf_frame_layout, rendering/mod.rs:563-651): a list of dicts with the plane's
+    pixel type name, width, height, `yuvi` index list and value limit."""
+    out = (abi.PlaneSpec * abi.FRAME_MAX_PLANES)(); n = C.c_size_t()
+    rc = abi.load_library().gf_frame_layout(abi.FRAME_FORMATS[format], width, height, out, C.byref(n))
+    if rc != 0:
+        raise GyroflowCoreError(rc, "gf_frame_layout")
+    return [dict(pixel_type=PIXEL_TYPE_NAMES[out[i].pixel_type], width=out[i].width, height=out[i].height,
+                 ind=tuple(out[i].ind[:out[i].n_ind]), max_value=float(out[i].max_value)) for i in range(n.value)]
+
+
+def background_for_plane(pixel_type: str, rgba, ind, is_limited: bool):
+    """PixelType::from_rgb_color (pixel_formats.rs:23-48): one plane's background from the RGBA colour (gf_background_for_plane)."""
+    v = (C.c_float * 4)(*[float(x) for x in rgba]); o = (C.c_float * 4)()
+    ia = (C.c_int32 * 4)(*(list(ind) + [0] * (4 - len(ind))))
+    rc = abi.load_library().gf_background_for_plane(abi.PIXEL_TYPES[pixel_type][0], v, ia, len(ind), int(is_limited), o)
+    if rc != 0:
+        raise GyroflowCoreError(rc, "gf_background_for_plane")
+    return np.array(o[:], dtype=np.float32)

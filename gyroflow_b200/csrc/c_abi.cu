@@ -372,7 +372,8 @@ GF_API size_t gf_abi_struct_size(int which) {
     case 0: return sizeof(gf_kernel_params);  case 1: return sizeof(gf_buffer_desc);    case 2: return sizeof(gf_compute_params);
     case 3: return sizeof(gf_camera_stab);    case 4: return sizeof(gf_keyframe_track); case 5: return sizeof(gf_stab_config);
     case 6: return sizeof(gf_queue_config);   case 7: return sizeof(gf_lens_data);
-    case 8: return sizeof(gf_mesh_f64);       default: return 0;
+    case 8: return sizeof(gf_mesh_f64);       case 9: return sizeof(gf_plane_spec);
+    default: return 0;
     }
 }
 GF_API const char* gf_cuda_backend_name(void) { return "CUDA"; }
@@ -906,21 +907,32 @@ GF_API int gf_cuda_generate_stmap(gf_cuda_gyro* g, const gf_compute_params* cp_u
 
 // Planes of one frame that share their geometry (GBRAPF32's four R32f planes, the U and V planes of planar YUV, ...):
 // every KernelParams field except plane_index and background must agree, as must buffer sizes, strides and rects.
-static bool planes_share_geometry(const gf_kernel_params* p, const gf_buffer_desc* in, const gf_buffer_desc* out, size_t n) {
-    for (size_t i = 1; i < n; ++i) {
-        gf_kernel_params a = p[0], b = p[i];
-        a.plane_index = b.plane_index = 0;
-        memset(a.background, 0, sizeof(a.background)); memset(b.background, 0, sizeof(b.background));
-        if (memcmp(&a, &b, sizeof(a)) != 0) return false;
-        const gf_buffer_desc* d[2][2] = {{&in[0], &in[i]}, {&out[0], &out[i]}};
-        for (auto& q : d) {
-            if (q[0]->width != q[1]->width || q[0]->height != q[1]->height || q[0]->stride != q[1]->stride || q[0]->len != q[1]->len ||
-                q[0]->has_rect != q[1]->has_rect || memcmp(q[0]->rect, q[1]->rect, sizeof(q[0]->rect)) != 0 ||
-                q[0]->has_rotation != q[1]->has_rotation || q[0]->rotation != q[1]->rotation || q[0]->kind != q[1]->kind) return false;
-        }
+static bool same_plane_geometry(const gf_kernel_params& pa, const gf_buffer_desc& ia, const gf_buffer_desc& oa,
+                                const gf_kernel_params& pb, const gf_buffer_desc& ib, const gf_buffer_desc& ob) {
+    gf_kernel_params a = pa, b = pb;
+    a.plane_index = b.plane_index = 0;
+    memset(a.background, 0, sizeof(a.background)); memset(b.background, 0, sizeof(b.background));
+    if (memcmp(&a, &b, sizeof(a)) != 0) return false;
+    const gf_buffer_desc* d[2][2] = {{&ia, &ib}, {&oa, &ob}};
+    for (auto& q : d) {
+        if (q[0]->width != q[1]->width || q[0]->height != q[1]->height || q[0]->stride != q[1]->stride || q[0]->len != q[1]->len ||
+            q[0]->has_rect != q[1]->has_rect || memcmp(q[0]->rect, q[1]->rect, sizeof(q[0]->rect)) != 0 ||
+            q[0]->has_rotation != q[1]->has_rotation || q[0]->rotation != q[1]->rotation || q[0]->kind != q[1]->kind) return false;
     }
     return true;
 }
+static bool planes_share_geometry(const gf_kernel_params* p, const gf_buffer_desc* in, const gf_buffer_desc* out, size_t n) {
+    for (size_t i = 1; i < n; ++i) if (!same_plane_geometry(p[0], in[0], out[0], p[i], in[i], out[i])) return false;
+    return true;
+}
+} // extern "C"
+
+bool gf_internal_same_plane_geometry(const gf_kernel_params* pa, const gf_buffer_desc* ia, const gf_buffer_desc* oa,
+                                     const gf_kernel_params* pb, const gf_buffer_desc* ib, const gf_buffer_desc* ob) {
+    return same_plane_geometry(*pa, *ia, *oa, *pb, *ib, *ob);
+}
+
+extern "C" {
 
 GF_API int gf_cuda_undistort_planes_dev(gf_cuda_ctx* ctx, size_t n_planes, const gf_buffer_desc* in, const gf_buffer_desc* out,
                                         const gf_kernel_params* params, const float* matrices_dev, size_t matrix_rows,

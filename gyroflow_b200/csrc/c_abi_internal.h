@@ -12,6 +12,10 @@ int gf_internal_run_frame(gf_cuda_ctx* ctx, const gf_buffer_desc* in, const gf_b
                           const float* matrices_dev, size_t matrix_rows, const float* mesh_dev, size_t mesh_len,
                           const uint32_t* table_flags_dev, void* cu_stream, uint64_t* checksum_dev);
 
+// Can two planes of one frame share one coordinate pass (gf_cuda_undistort_planes_dev_flagged fuses planes for which this holds)?
+bool gf_internal_same_plane_geometry(const gf_kernel_params* pa, const gf_buffer_desc* ia, const gf_buffer_desc* oa,
+                                     const gf_kernel_params* pb, const gf_buffer_desc* ib, const gf_buffer_desc* ob);
+
 // Preview overlays (overlay.cu): draw_pixel + draw_safe_area of opencl_undistort.cl:109-154 as a pass over a DEVICE buffer.
 // count / scalar: channels and scalar kind (0 u8, 1 u16, 2 f32, 3 f16) of the pixel type.
 int gf_internal_draw_overlays(void* cu_stream, uint8_t* buf_dev, size_t len, int width, int height, int stride, const gf_kernel_params* p,

@@ -93,6 +93,83 @@ class RenderQueue:
         except Exception: pass
 
 
+class FrameRenderQueue:
+    """A render queue over whole decoder frames (gf_cuda_queue_create_frame): every submission is all planes of one frame of `format`
+    (NV12, P010LE, YUV420P, ... — abi.FRAME_FORMATS), with one producer launch per frame and each plane's KernelParams set the way the
+    reference's per-plane closures set them (rendering/mod.rs:483-548): value limit, background converted for the plane, plane_index,
+    per-frame FILL_WITH_BACKGROUND.  `stab` describes the whole frame; its pixel_type is ignored.  in_protos / out_protos: one
+    BufferDescription per plane in the order of frame_layout(format, ...)."""
+
+    def __init__(self, compute_params, stab: abi.StabConfig, format: str, distortion_model: str, digital_lens, in_protos, out_protos,
+                 limited_range=False, device=0, depth=4, pin_numa=True, checksum=False):
+        self._lib = abi.load_library()
+        self.cp = compute_params
+        cfg = abi.QueueConfig()
+        cfg.device = device
+        cfg.distortion_model = abi.LENS[distortion_model]
+        cfg.digital_lens = abi.LENS[digital_lens] if digital_lens else 0
+        cfg.depth, cfg.pin_numa, cfg.checksum = depth, int(pin_numa), int(checksum)
+        cfg.stab = stab
+        self.depth = depth
+        self.in_flight = 0
+        self.n_planes = len(in_protos)
+        h = C.c_void_p()
+        i = (abi.BufferDesc * self.n_planes)(*[b.to_c() for b in in_protos])
+        o = (abi.BufferDesc * len(out_protos))(*[b.to_c() for b in out_protos])
+        rc = self._lib.gf_cuda_queue_create_frame(C.byref(h), C.byref(cfg), C.byref(compute_params.c), abi.FRAME_FORMATS[format],
+                                                  int(limited_range), self.n_planes, i, o)
+        if rc != 0:
+            raise GyroflowCoreError(rc, "gf_cuda_queue_create_frame: " + (self._lib.gf_cuda_last_error(None) or b"").decode())
+        self._h = h
+
+    def _err(self, rc, what):
+        return GyroflowCoreError(rc, what + ": " + (self._lib.gf_cuda_queue_last_error(self._h) or b"").decode())
+
+    def submit(self, frame: int, timestamp_ms: float, planes, mesh=None, fill_with_background=False):
+        """Enqueue one frame; `planes` is a list of Buffers, one per plane.  The queue must have a free slot."""
+        n = len(planes)
+        i = (abi.BufferDesc * max(n, 1))(*[b.input.to_c() for b in planes])
+        o = (abi.BufferDesc * max(n, 1))(*[b.output.to_c() for b in planes])
+        m = None if mesh is None else np.ascontiguousarray(mesh, dtype=np.float32)
+        rc = self._lib.gf_cuda_queue_submit_frame(self._h, frame, timestamp_ms, n, i, o, m.ctypes.data if m is not None and m.size else None,
+                                                  m.size if m is not None else 0, int(bool(fill_with_background)))
+        if rc != 0:
+            raise self._err(rc, "gf_cuda_queue_submit_frame")
+        self.in_flight += 1
+
+    def wait(self):
+        """Block until the oldest in-flight frame is finished; returns (frame, (checksum per plane))."""
+        f = C.c_size_t(); s = (C.c_uint64 * self.n_planes)()
+        rc = self._lib.gf_cuda_queue_wait_frame(self._h, C.byref(f), s, self.n_planes)
+        if rc != 0:
+            raise self._err(rc, "gf_cuda_queue_wait_frame")
+        self.in_flight -= 1
+        return int(f.value), tuple(int(v) for v in s)
+
+    def render(self, frames, timestamp_of, planes_of, mesh_of=None, fill_of=None):
+        """Run `frames` through the queue keeping it full; returns {frame: (checksum per plane)} in frame order."""
+        out = {}
+        for f in frames:
+            if self.in_flight == self.depth:
+                k, v = self.wait(); out[k] = v
+            self.submit(f, timestamp_of(f), planes_of(f), mesh_of(f) if mesh_of else None, fill_of(f) if fill_of else False)
+        while self.in_flight:
+            k, v = self.wait(); out[k] = v
+        return dict(sorted(out.items()))
+
+    @property
+    def launch_count(self):
+        return int(self._lib.gf_cuda_queue_launches(self._h))
+
+    def close(self):
+        if getattr(self, "_h", None):
+            self._lib.gf_cuda_queue_destroy(self._h); self._h = None
+
+    def __del__(self):
+        try: self.close()
+        except Exception: pass
+
+
 def checksum_host(buf: np.ndarray) -> int:
     """The queue's per-frame checksum on the host: sum(word[i] * (2 i + 1)) mod 2^64 over the buffer's 32-bit words."""
     w = np.ascontiguousarray(buf).view(np.uint8).reshape(-1)

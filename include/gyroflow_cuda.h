@@ -203,7 +203,7 @@ GF_API int         gf_cuda_device_name(int device, char* buf, size_t buf_len);  
 GF_API int         gf_cuda_supports(const gf_buffer_desc* in, const gf_buffer_desc* out); /* is_buffer_supported opencl.rs:451 */
 GF_API const char* gf_cuda_version(void);
 /* sizeof() of the structs that cross this ABI, for binding generators and their tests: 0 gf_kernel_params, 1 gf_buffer_desc,
- * 2 gf_compute_params, 3 gf_camera_stab, 4 gf_keyframe_track, 5 gf_stab_config, 6 gf_queue_config, 7 gf_lens_data, 8 gf_mesh_f64; 0 for any other index. */
+ * 2 gf_compute_params, 3 gf_camera_stab, 4 gf_keyframe_track, 5 gf_stab_config, 6 gf_queue_config, 7 gf_lens_data, 8 gf_mesh_f64, 9 gf_plane_spec; 0 for any other index. */
 GF_API size_t gf_abi_struct_size(int which);
 
 /* ---- lens plugin surface: DistortionModel::from_name / id  distortion_models/mod.rs:79-90 -- */
@@ -533,6 +533,60 @@ GF_API int      gf_cuda_queue_drain(gf_cuda_queue* q);                          
 GF_API uint64_t gf_cuda_queue_launches(gf_cuda_queue* q);                                          /* warp + producer (+ checksum) kernels launched */
 GF_API void     gf_cuda_queue_destroy(gf_cuda_queue* q);
 GF_API const char* gf_cuda_queue_last_error(gf_cuda_queue* q);
+
+/* ------------------------------------------------------------------------------------------
+ * Decoder frames — the plane table of rendering/mod.rs:563-651 (create_planes_proc!, :483-548).  A frame of one of these formats
+ * is rendered plane by plane; every plane has its own pixel type, size, `yuvi` index list and value limit, copied from the table as
+ * written (GBRAPF32's [2],[0],[1],[3] order and limit 255, P0xx at 65535, the big-endian RGB48BE / RGBA64BE rows on RGB16 / RGBA16).
+ * ---------------------------------------------------------------------------------------- */
+enum {
+    GF_FRAME_NV12 = 0, GF_FRAME_NV21,
+    GF_FRAME_P010LE, GF_FRAME_P016LE, GF_FRAME_P210LE, GF_FRAME_P216LE, GF_FRAME_P410LE, GF_FRAME_P416LE,
+    GF_FRAME_YUV420P, GF_FRAME_YUVJ420P,
+    GF_FRAME_YUV420P10LE, GF_FRAME_YUV420P12LE, GF_FRAME_YUV420P14LE, GF_FRAME_YUV420P16LE,
+    GF_FRAME_YUV422P10LE, GF_FRAME_YUV422P12LE, GF_FRAME_YUV422P14LE, GF_FRAME_YUV422P16LE,
+    GF_FRAME_YUV444P10LE, GF_FRAME_YUV444P12LE, GF_FRAME_YUV444P14LE, GF_FRAME_YUV444P16LE,
+    GF_FRAME_YUVA444P10LE, GF_FRAME_YUVA444P12LE, GF_FRAME_YUVA444P16LE,
+    GF_FRAME_GBRAPF32LE, GF_FRAME_GBRPF32LE, GF_FRAME_AYUV64LE,
+    GF_FRAME_RGB24, GF_FRAME_RGBA, GF_FRAME_RGB48BE, GF_FRAME_RGBA64BE,
+    GF_FRAME_COUNT
+};
+#define GF_FRAME_MAX_PLANES 4
+typedef struct gf_plane_spec {
+    int32_t pixel_type;                 /* GF_PIX_* ($t) */
+    int32_t width, height;              /* the plane's size in its own pixels (zero_copy::get_plane_size): ffmpeg's plane_width / plane_height */
+    int32_t n_ind;                      /* length of the `yuvi` list ($yuvi), 0..4 */
+    int32_t ind[4];
+    float   max_value;                  /* $max_val: pixel_value_limit and max_pixel_value of the plane (:532-533) */
+} gf_plane_spec;
+/* Host only.  Fills out[0..*n) for a width x height frame (chroma planes -((-w) >> log2_chroma_w) wide, the same rule for the height;
+ * GBR(A)PF32 planes all take plane 0's size).  `out` has room for GF_FRAME_MAX_PLANES.  GF_ERR_BAD_PARAMS for an unknown format or a
+ * non-positive size. */
+GF_API int gf_frame_layout(int format, int32_t width, int32_t height, gf_plane_spec* out, size_t* n);
+/* PixelType::from_rgb_color (pixel_formats.rs:23-48 and the per-type impls): the background colour of one plane.  `rgb` is
+ * ComputeParams.background (RGBA, 0..1); YUV planes go through rgb_to_yuv (Rec.709, clamped, then remapped to 16-235 / 16-240 when
+ * is_limited) in f32 with the reference's operation order.  GF_ERR_BAD_PARAMS if the pixel type needs more indices than n_ind or an
+ * index is outside 0..3. */
+GF_API int gf_background_for_plane(int pixel_type, const float rgb[4], const int32_t* ind, size_t n_ind, int is_limited, float out[4]);
+
+/* Render queue over whole decoder frames — replaces the per-plane closures of rendering/mod.rs:483-548 and the plane loop of
+ * :657-661.  One queue = one format: cfg->stab describes the whole frame (size, output size, interpolation, flags, RGB background;
+ * its pixel_type is ignored), `is_limited_range` selects the background conversion (:506).  in_protos / out_protos: one prototype
+ * buffer per plane, in the order of gf_frame_layout.  Each slot holds one device table + verdict word, one warp context per distinct
+ * pixel type and (HOST buffers) device staging per plane.  Per submitted frame, on the slot's stream and without a host sync:
+ *     one gf_cuda_frame_transform_dev_flagged  ->  [mesh H2D]  ->  [plane H2D]  ->  per plane get_frame_transform_at + the plane's value
+ *     limit, converted background, plane_index = position in the list, FILL_WITH_BACKGROUND when asked (:531-541)  ->  warp (planes of
+ *     one pixel type and equal geometry share one coordinate pass)  ->  [one checksum launch over every plane]  ->  [plane D2H]
+ * gf_cuda_queue_submit_frame: GF_ERR_BAD_PARAMS for a wrong plane count or a full queue, GF_ERR_SIZE_MISMATCH when a plane's buffer size
+ * differs from the layout.  gf_cuda_queue_wait_frame writes min(n_checksums, n_planes) checksums, one per plane (zeros when
+ * cfg->checksum is 0); over HOST planes the sums cover the device copy, whose row padding is zero unless a plane was uploaded whole.
+ * gf_cuda_queue_submit refuses a frame queue and gf_cuda_queue_submit_frame a single-buffer queue; the wait, drain, launch-count,
+ * destroy and last-error calls work on both. */
+GF_API int      gf_cuda_queue_create_frame(gf_cuda_queue** out, const gf_queue_config* cfg, const gf_compute_params* cp, int format,
+                                           int is_limited_range, size_t n_planes, const gf_buffer_desc* in_protos, const gf_buffer_desc* out_protos);
+GF_API int      gf_cuda_queue_submit_frame(gf_cuda_queue* q, size_t frame, double timestamp_ms, size_t n_planes, const gf_buffer_desc* in,
+                                           const gf_buffer_desc* out, const float* mesh, size_t mesh_len, int fill_with_background);
+GF_API int      gf_cuda_queue_wait_frame(gf_cuda_queue* q, size_t* out_frame, uint64_t* out_checksums, size_t n_checksums);
 
 /* Bind the calling thread to the CPUs of the NUMA node the GPU hangs off (/sys/bus/pci/devices/<bdf>/local_cpulist), so that
  * page-locked staging allocated afterwards — by this library or by the caller — is node-local and the copy threads do not cross

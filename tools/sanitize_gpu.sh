@@ -1,6 +1,7 @@
 #!/bin/sh
 # Runs ON THE GPU BOX: compute-sanitizer memcheck + racecheck + initcheck-free runs over the smoke case, one filtered-pre-pass frame with
 # deferred pairs, one two-pass (Lanczos4) case, one fused multi-plane case and a short render-queue run.  Logs -> gpurun_out/sanitizer_*.log
+# The Python cases end with a short NV12 frame queue over page-locked HOST planes.
 cat > /tmp/san_cases.py <<'PY'
 import sys, numpy as np
 sys.path.insert(0, ".")
@@ -24,6 +25,14 @@ src = torch.zeros((180, p.stride), dtype=torch.uint8, device="cuda"); outs = [to
 mk = lambda f: g.Buffers(g.BufferDescription((320, 180, p.stride), src.data_ptr(), length=src.numel()), g.BufferDescription((320, 180, p.output_stride), outs[f].data_ptr(), length=outs[f].numel()))
 q = g.RenderQueue(cp, st, "opencv_fisheye", None, mk(0).input, mk(0).output, depth=3, checksum=True)
 print(q.render(range(6), lambda f: 100.0 + 16.6 * f, mk)); q.close()
+# a small NV12 frame queue with page-locked HOST planes (two warp contexts, one producer launch, one checksum launch per frame)
+lay = g.frame_layout("NV12", 321, 181); st = g.stab_config(synth.base_kernel_params(321, 181), "Luma8")
+cp = g.ComputeParams(synth.base_kernel_params(321, 181), org, sm, fov_scale=1.5)
+hb = [[(torch.from_numpy(synth.synthetic_frame(l["width"], l["height"], l["pixel_type"], frame=f, stride=512)).pin_memory(),
+        torch.zeros((l["height"], 512), dtype=torch.uint8).pin_memory()) for l in lay] for f in range(4)]
+pk = lambda f: [g.Buffers(g.BufferDescription((l["width"], l["height"], 512), a.numpy()), g.BufferDescription((l["width"], l["height"], 512), b.numpy())) for l, (a, b) in zip(lay, hb[f])]
+fq = g.FrameRenderQueue(cp, st, "NV12", "opencv_fisheye", None, [x.input for x in pk(0)], [x.output for x in pk(0)], depth=2, checksum=True)
+print(fq.render(range(4), lambda f: 100.0 + 16.6 * f, pk, fill_of=lambda f: f == 2)); fq.close()
 print("sanitizer cases done")
 PY
 for tool in memcheck racecheck; do
